@@ -1,6 +1,6 @@
 """bench.py — nucleotides/sec of the Evo-1 7B forward on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 8k|131k|1k|32k|gen] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 8k|131k|1k|32k|gen] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload "8k" (default, BASELINE.json configs[1]): evo-1-8k-base scoring forward, batch 8 x
 8192 nt of synthetic uniform ACGT (+BOS => L = 8193), bf16, random-init weights of the 7B
@@ -13,6 +13,8 @@ collective (weak scaling); "131k" runs the sequence-parallel forward instead.
 --impl reference: the reference's own CPU implementation of the path.  stripedhyena==0.2.2 is
 not installable offline, so this arm times the oracle restatement (kind "port") on the host
 cores, rank 0 only, on a bounded sample of the same workload.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the timed path returned in its last step as DIR/<name>.npy
+(see dump_outputs), so that two builds can be compared output for output on the same seeded inputs and weights.
 """
 from __future__ import annotations
 
@@ -52,6 +54,25 @@ def measured_peaks():
         p = json.load(open(path))
         return {"hbm_gbs": p["hbm_gbs"], "bf16_tflops": p["bf16_tflops"], "bf16_tflops_sustained": p.get("bf16_tflops_sustained", p["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_ARRAY_BYTES = 16 << 20        # per array; a path returns at most two arrays, so a dump stays well under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as `path`/<name>.npy: float32, or float64 for values the API hands back as host floats.  An array
+    over DUMP_ARRAY_BYTES keeps a fixed sample of its rows (rows = all but the last dimension, chosen with seed 0, kept in
+    row order), so the same shape always yields the same rows."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a, dtype=np.float64)
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            rows = a.reshape(-1, a.shape[-1])
+            keep = DUMP_ARRAY_BYTES // (rows.shape[1] * a.itemsize)
+            a = rows[np.sort(np.random.default_rng(0).choice(rows.shape[0], size=keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def ncu_traffic(pattern, workload):
@@ -223,16 +244,17 @@ def _max_over_ranks(x, world, dev):
 
 def time_steps(fwd, steps, world, dev):
     """EXACTLY `steps` calls of fwd, CUDA events on the launch stream, barrier + synchronize on both sides.
-    No per-kernel instrumentation runs inside this region."""
+    No per-kernel instrumentation runs inside this region.  Returns (max ms over ranks, per-rank ms, last step's result)."""
     import torch
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    out = None
     _barrier(world)
     e0.record()
     for _ in range(steps):
-        fwd()
+        out = fwd()
     e1.record()
     _barrier(world)
-    return _max_over_ranks(e0.elapsed_time(e1), world, dev)
+    return (*_max_over_ranks(e0.elapsed_time(e1), world, dev), out)
 
 
 def kernel_breakdown(model, fwd, n, world):
@@ -317,7 +339,7 @@ def sp131k_record(model8k, world, rank, dev, steps, warmup, peaks):
         fwd = lambda: model(ids_full)[0]
     for _ in range(warmup):
         fwd()
-    ms, per_rank = time_steps(fwd, steps, world, dev)
+    ms, per_rank, _ = time_steps(fwd, steps, world, dev)
     by, prof_ms = kernel_breakdown(model, fwd, 1, world)
     rec = {"workload": wl["desc"], "value": wl["batch"] * wl["nt"] * steps / (ms / 1e3), "unit": "nt/s", "ms_per_step": ms / steps, "steps": steps, "warmup": warmup,
            "parallelism": f"sp{world}", "scaling": "strong", "per_rank_ms_per_step": [v / steps for v in per_rank], "tokens_per_rank": shard}
@@ -364,7 +386,7 @@ def sweep_record(model8k, dev, steps=3, warmup=1):
         fwd = lambda: m(ids)
         for _ in range(warmup):
             fwd()
-        ms, _ = time_steps(fwd, steps, 1, dev)
+        ms, _, _ = time_steps(fwd, steps, 1, dev)
         out[key] = {"workload": wl["desc"], "value": wl["batch"] * wl["nt"] * steps / (ms / 1e3), "unit": "nt/s", "ms_per_step": ms / steps, "steps": steps, "warmup": warmup}
         del ids
         torch.cuda.empty_cache()
@@ -407,9 +429,11 @@ def bench_ours(args, wl):
     lib = _lib.lib()
     lib.evo_reset_launch_count()
     with ClockSampler(local) as clocks:
-        ms, per_rank_ms = time_steps(fwd, steps, world, dev)
+        ms, per_rank_ms, last = time_steps(fwd, steps, world, dev)
     launches = lib.evo_launch_count()
     value = tokens_per_step_job * steps / (ms / 1e3)
+    dumped = {"logits": last[0] if isinstance(last, tuple) else last}
+    del last
 
     # ---- separate pass: per-kernel events for the rooflines (not part of `value`)
     by, prof_ms = kernel_breakdown(model, fwd, 2, world)
@@ -429,6 +453,10 @@ def bench_ours(args, wl):
         e2e = {"value": tokens_per_step_job * steps / dt, "unit": "nt/s",
                "h2d_bytes_per_step": wl["batch"] * L1 * 8, "d2h_bytes_per_step": wl["batch"] * wl["nt"] * 4,
                "api": "evo_b200.score_sequences(list[str]) -> list[float]"}
+        dumped["e2e_scores"] = scores
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumped)
+    del dumped
 
     peaks = measured_peaks()
     sub = {}
@@ -473,11 +501,12 @@ def bench_ours(args, wl):
         dist.destroy_process_group()
 
 
-def generate_record(model, dev, peaks, steps=64, warmup=4, n_new=None, world=1, rank=0):
+def generate_record(model, dev, peaks, steps=64, warmup=4, n_new=None, world=1, rank=0, outputs=None):
     """BASELINE.json configs[3]: cached generation, batch 16, prompt 4096 nt, greedy.  One step = one new nucleotide per
     sequence through the L == 1 path (recurrent Hyena state + KV cache).
     value = generated nt/s with the state resident on the GPU; e2e = evo_b200.generate() from prompt strings to generated
-    strings, the 4096-nt prefill and `n_new` decode steps included."""
+    strings, the 4096-nt prefill and `n_new` decode steps included.  `outputs` (a dict) receives the last timed step's
+    logits and greedy next tokens."""
     import torch
     import evo_b200
     from evo_b200 import _lib, CharLevelTokenizer
@@ -494,8 +523,8 @@ def generate_record(model, dev, peaks, steps=64, warmup=4, n_new=None, world=1, 
     state = {"nxt": logits[:, -1].argmax(-1, keepdim=True), "d": d}
 
     def step():
-        lg, state["d"] = model(state["nxt"], inference_params_dict=state["d"])
-        state["nxt"] = lg[:, -1].argmax(-1, keepdim=True)
+        state["lg"], state["d"] = model(state["nxt"], inference_params_dict=state["d"])
+        state["nxt"] = state["lg"][:, -1].argmax(-1, keepdim=True)
         state["d"]["mha"].seqlen_offset += 1
         state["d"]["hyena"].seqlen_offset += 1
 
@@ -515,6 +544,8 @@ def generate_record(model, dev, peaks, steps=64, warmup=4, n_new=None, world=1, 
     launches = lib.evo_launch_count() - n0
     if world > 1:
         ms, _ = _max_over_ranks(ms, world, dev)
+    if outputs is not None:
+        outputs.update(logits=state["lg"], next_token=state["nxt"])
     del state, d, logits
     torch.cuda.empty_cache()
     # end to end: prompts as strings -> generated strings through the reference-shaped API (prefill + n_new steps)
@@ -553,8 +584,12 @@ def bench_generate(args, wl):
     steps = args.steps if args.steps is not None else 64
     warmup = max(3, args.warmup if args.warmup is not None else 4)
     model = load_checkpoint(wl["model"], device=dev, random_init=True, seed=0)
+    dumped = {}
     with ClockSampler(local) as clocks:
-        rec = generate_record(model, dev, measured_peaks(), steps=steps, warmup=warmup, n_new=args.gen_tokens, world=world, rank=rank)
+        rec = generate_record(model, dev, measured_peaks(), steps=steps, warmup=warmup, n_new=args.gen_tokens, world=world, rank=rank, outputs=dumped)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumped)
+    del dumped
     if rank == 0:
         out = {"metric": rec.pop("metric"), "value": rec.pop("value"), "unit": rec.pop("unit"), "n_gpus": world, "steps": steps, "warmup": warmup,
                "ms_per_step": rec.pop("ms_per_step"), "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
@@ -580,7 +615,11 @@ def main():
     ap.add_argument("--no-gen", action="store_true", help="skip the cached-generation sub-record")
     ap.add_argument("--sub-steps", type=int, default=3, help="timed steps of the 131k sub-record")
     ap.add_argument("--gen-tokens", type=int, default=None, help="new tokens of the end-to-end generate() run (default: 4096 = BASELINE configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (float32/float64, < 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         bench_reference(args, wl)

@@ -1,20 +1,21 @@
-"""Generates tests/golden/reference_host.{json,npz}: outputs of the REFERENCE'S OWN host code, run in the build container.
+"""Generates tests/golden/reference_host.{json,npz}: outputs of the REFERENCE'S OWN host code, run on CPU.
 
-What is pinned.  /root/reference/evo/{tokenizer,scoring,generation,models}.py are the reference for everything on either
+What is pinned.  evo/{tokenizer,scoring,generation,models}.py of the reference checkout are the reference for everything on either
 side of the model call (SURVEY.md 8b, 8f-1..4): tokenisation, batch preparation, the logits -> log-likelihood / entropy
 reductions, the generation loop's state protocol (which slices of the prompt the model sees and which `seqlen_offset` it is
 handed at every call, quirks Q1-Q4 included) and checkpoint ingest (HF repo / revision, 'backbone.' strip, tied unembed,
 YAML config, strict load, dtype policy call order).  Those files import `stripedhyena`, which does not exist here
 (SURVEY.md 0.1) -- so this script registers a stand-in `stripedhyena` package whose `StripedHyena` is a recorder, whose
 `sample` is flash_attn.utils.generation.sample (installed here; the function stripedhyena/sample.py copies) and whose `dotdict`
-is a plain attribute dict, imports the reference's modules UNMODIFIED from /root/reference, and drives them on CPU with the
-oracle model (oracle/stripedhyena_oracle.py) standing where the real model would.
+is a plain attribute dict, imports the reference's modules UNMODIFIED from the checkout, and drives them on CPU with the
+oracle model (oracle/stripedhyena_oracle.py) standing where the real model would.  The bf16 oracle's logits are stored too:
+a bf16 matmul on CPU rounds differently with and without AMX, so the test replays them instead of recomputing them.
 
 What is NOT pinned by this: the model arithmetic (the oracle stays a restatement; "parity unpinned" in its header stands).
 The fixtures pin the host layer: tests/test_reference_host_golden.py runs evo_b200's host code over the SAME oracle model and
 must reproduce every id, call, string and score; the GPU tests compare the CUDA path's scores with the fp64 numbers.
 
-    python tests/golden/make_reference_host_golden.py        (build container only: needs /root/reference)
+    python tests/golden/make_reference_host_golden.py <path of the reference checkout>
 """
 import hashlib
 import json
@@ -28,7 +29,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.normpath(os.path.join(HERE, "..", ".."))
-REFERENCE = "/root/reference"
+REFERENCE = None          # the reference checkout, from the command line
 sys.path.insert(0, ROOT)
 
 from oracle import stripedhyena_oracle as O  # noqa: E402
@@ -84,6 +85,7 @@ class OracleAsModel:
     def __init__(self, cfg, sd, dtype):
         self.m = O.OracleStripedHyena(cfg, sd, dtype)
         self.calls = []
+        self.logits = []
 
     def eval(self):
         return self
@@ -94,7 +96,9 @@ class OracleAsModel:
     def __call__(self, x, inference_params_dict=None):
         d = inference_params_dict
         self.calls.append([list(x.shape), None if d is None else int(d["mha"].seqlen_offset), None if d is None else int(d["hyena"].seqlen_offset)])
-        return self.m(x, d)
+        out = self.m(x, d)
+        self.logits.append(out[0])
+        return out
 
 
 def tiny():
@@ -139,8 +143,12 @@ def scoring_cases(RS, RT, arrays):
             model = OracleAsModel(cfg, sd, dtype)
             out[f"score_{red}_{name}"] = [float(s) for s in RS.score_sequences(SEQS, model, tok, reduce_method=red, device="cpu")]
             out[f"score_calls_{name}"] = model.calls
+        if dtype == torch.bfloat16:
+            arrays["score_logits_bf16"] = model.logits[0].float().numpy()       # exact: bf16 values fit in fp32
         model = OracleAsModel(cfg, sd, dtype)
         ent = RS.positional_entropies(SEQS, model, tok, device="cpu")
+        if dtype == torch.bfloat16:
+            assert np.array_equal(model.logits[0].float().numpy(), arrays["score_logits_bf16"])    # one batch feeds both reductions
         for k, e in enumerate(ent):
             arrays[f"entropy_{name}_{k}"] = np.asarray(e, dtype=np.float32)
     try:
@@ -266,7 +274,7 @@ def checkpoint_cases(RM):
 
 
 def _load_reference_script(name):
-    """A file under /root/reference/scripts as a module of its own (the repo has a `scripts` package of the same name)."""
+    """A file under the reference's scripts/ as a module of its own (the repo has a `scripts` package of the same name)."""
     import importlib.util
     spec = importlib.util.spec_from_file_location("reference_scripts_" + name, os.path.join(REFERENCE, "scripts", name + ".py"))
     mod = importlib.util.module_from_spec(spec)
@@ -374,8 +382,10 @@ def bucketing_cases():
 
 
 def main():
-    if not os.path.isdir(os.path.join(REFERENCE, "evo")):
-        raise SystemExit("needs /root/reference (build container only)")
+    global REFERENCE
+    if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "evo")):
+        raise SystemExit("usage: make_reference_host_golden.py <path of the reference checkout (the directory holding evo/)>")
+    REFERENCE = os.path.realpath(sys.argv[1])
     install_stand_in()
     sys.path.insert(0, REFERENCE)
     import evo.generation as RG
