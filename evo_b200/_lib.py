@@ -66,6 +66,14 @@ class LoopParams(C.Structure):
                 ("seed", C.c_uint64), ("step0", C.c_int64)]
 
 
+class RaggedLoopParams(C.Structure):
+    _fields_ = [("n_forced", C.c_void_p), ("n_out", C.c_void_p), ("start", C.c_void_p),
+                ("forced", C.c_void_p), ("forced_stride", C.c_int64),
+                ("picked", C.c_void_p), ("kept_logits", C.c_void_p), ("out_cols", C.c_int64),
+                ("top_k", C.c_int32), ("top_p", C.c_float), ("temperature", C.c_float),
+                ("seed", C.c_uint64)]
+
+
 # name -> (restype, argtypes); every symbol include/evo_b200.h declares
 SIGNATURES = {
     "evo_last_error": (C.c_char_p, []),
@@ -81,6 +89,8 @@ SIGNATURES = {
     "evo_set_pdl": (C.c_int, [C.c_int]),
     "evo_hyena_fwd_workspace": (C.c_size_t, [C.POINTER(HyenaParams)]),
     "evo_hyena_fwd": (C.c_int, [C.POINTER(HyenaParams), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "evo_hyena_fwd_ragged_workspace": (C.c_size_t, [C.POINTER(HyenaParams)]),
+    "evo_hyena_fwd_ragged": (C.c_int, [C.POINTER(HyenaParams), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "evo_hyena_step": (C.c_int, [C.c_void_p] * 9 + [C.c_int] * 4 + [C.c_void_p]),
     "evo_hyena_combine_states": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "evo_peer_publish": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
@@ -94,10 +104,14 @@ SIGNATURES = {
     "evo_decode_qkv_prep": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p]),
     "evo_decode_attn_workspace": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "evo_decode_attn": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_float, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "evo_decode_qkv_prep_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p]),
+    "evo_decode_attn_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_float, C.c_void_p, C.c_size_t, C.c_void_p]),
     "evo_advance_position": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "evo_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_uint64, C.c_uint64, C.c_void_p]),
     "evo_sample_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "evo_advance_counters": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "evo_sample_step_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "evo_ragged_advance": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "evo_unembed_score_workspace": (C.c_size_t, [C.c_int64, C.c_int]),
     "evo_unembed_score": (C.c_int, [C.POINTER(ScoreParams), C.c_void_p]),
     "evo_tokenize_pad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p]),

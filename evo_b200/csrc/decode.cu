@@ -30,13 +30,16 @@ __global__ void gelu_gate_kernel(const bf16* __restrict__ t, bf16* __restrict__ 
 
 // L == 1: rotary on q,k at position *pos, k,v appended to the cache at row *pos.
 // qkv (B, 3, H, 128) in place; cos/sin tables indexed by absolute position.
+// ROWS: pos_ptr is a (B) vector and row b uses pos_ptr[b] (ragged batches); otherwise one position for the batch.
+template <bool ROWS>
 __global__ void decode_qkv_prep_kernel(bf16* __restrict__ qkv, bf16* __restrict__ cache, const bf16* __restrict__ cos, const bf16* __restrict__ sin,
                                        const long long* __restrict__ pos_ptr, int B, int H, long long max_seqlen) {
   pdl_launch_dependents(); pdl_wait();
-  const long long pos = *pos_ptr;
   int idx = blockIdx.x * blockDim.x + threadIdx.x;       // (b, h, i) i in [0, 64)
-  if (idx >= B * H * 64 || pos >= max_seqlen) return;
+  if (idx >= B * H * 64) return;
   int i = idx % 64, h = (idx / 64) % H, b = idx / (64 * H);
+  const long long pos = pos_ptr[ROWS ? b : 0];
+  if (pos < 0 || pos >= max_seqlen) return;
   const float c = __bfloat162float(cos[pos * 64 + i]), s = __bfloat162float(sin[pos * 64 + i]);
   bf16* q = qkv + ((long long)(b * 3 + 0) * H + h) * HD;
   bf16* k = qkv + ((long long)(b * 3 + 1) * H + h) * HD;
@@ -58,12 +61,13 @@ __global__ void decode_qkv_prep_kernel(bf16* __restrict__ qkv, bf16* __restrict_
 // V row per key), keeps an online-softmax state and a 128-wide fp32 accumulator in registers, and the
 // 128 partial states are merged through shared memory; splits are merged by the last kernel.
 constexpr int DT = 128;
+template <bool ROWS>
 __global__ void __launch_bounds__(DT) decode_attn_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ cache, float* __restrict__ part_o,
                                                          float* __restrict__ part_ml, const long long* __restrict__ pos_ptr,
                                                          int H, long long max_seqlen, int nsplit, float scale) {
   pdl_launch_dependents(); pdl_wait();
   const int h = blockIdx.x, b = blockIdx.y, sp = blockIdx.z, tid = threadIdx.x;
-  const long long nk = min(*pos_ptr + 1, max_seqlen);
+  const long long nk = min(pos_ptr[ROWS ? b : 0] + 1, max_seqlen);
   const long long per = (nk + nsplit - 1) / nsplit;
   const long long k0 = (long long)sp * per, k1 = min(nk, k0 + per);
   __shared__ float qs[HD];
@@ -139,6 +143,7 @@ constexpr int TK = 64;                 // keys per tile
 constexpr int AST = 3;                 // ring stages
 constexpr int TILE_BYTES = TK * HD * 2;          // 16 KB (K) + 16 KB (V) per stage
 constexpr int ATT2_SMEM = AST * 2 * TILE_BYTES + 1024;
+template <bool ROWS>
 __global__ void __launch_bounds__(160, 2) decode_attn_tma_kernel(const __grid_constant__ CUtensorMap tm, const bf16* __restrict__ qkv,
                                                                  float* __restrict__ part_o, float* __restrict__ part_ml,
                                                                  const long long* __restrict__ pos_ptr, int H, long long S, int nsplit, float scale) {
@@ -149,7 +154,7 @@ __global__ void __launch_bounds__(160, 2) decode_attn_tma_kernel(const __grid_co
   bf16* qb = reinterpret_cast<bf16*>(empty + AST);                   // 256 B
   float* red = reinterpret_cast<float*>(qb + HD);                      // [4][2] (m, l) then [4][128] o, overlaid on stage 0 after the loop
   const int h = blockIdx.x, b = blockIdx.y, sp = blockIdx.z, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const long long nk = min(*pos_ptr + 1, S);
+  const long long nk = min(pos_ptr[ROWS ? b : 0] + 1, S);
   long long per = (nk + nsplit - 1) / nsplit;
   per = (per + TK - 1) / TK * TK;                                      // splits start on tile boundaries
   const long long k0 = (long long)sp * per, k1 = min(nk, k0 + per);
@@ -275,22 +280,34 @@ extern "C" int evo_gelu_gate_interleaved(const void* t, void* out, int64_t M, in
   return check_launch("evo_gelu_gate_interleaved");
 }
 
+template <bool ROWS>
+static int decode_qkv_prep(const char* name, void* qkv, void* cache, const void* cos, const void* sin, const int64_t* pos,
+                           int B, int H, int hd, int64_t max_seqlen, void* stream) {
+  EVO_REQUIRE(hd == HD, "%s: head_dim %d unsupported", name, hd);
+  int n = B * H * 64;
+  EVO_CUDA(launch_pdl(decode_qkv_prep_kernel<ROWS>, dim3((n + 127) / 128), dim3(128), 0, (cudaStream_t)stream, (bf16*)qkv, (bf16*)cache, (const bf16*)cos, (const bf16*)sin,
+                      (const long long*)pos, B, H, max_seqlen));
+  return check_launch(name);
+}
+
 extern "C" int evo_decode_qkv_prep(void* qkv, void* cache, const void* cos, const void* sin, const int64_t* pos,
                                    int B, int H, int hd, int64_t max_seqlen, void* stream) {
-  EVO_REQUIRE(hd == HD, "evo_decode_qkv_prep: head_dim %d unsupported", hd);
-  int n = B * H * 64;
-  EVO_CUDA(launch_pdl(decode_qkv_prep_kernel, dim3((n + 127) / 128), dim3(128), 0, (cudaStream_t)stream, (bf16*)qkv, (bf16*)cache, (const bf16*)cos, (const bf16*)sin,
-                      (const long long*)pos, B, H, max_seqlen));
-  return check_launch("evo_decode_qkv_prep");
+  return decode_qkv_prep<false>("evo_decode_qkv_prep", qkv, cache, cos, sin, pos, B, H, hd, max_seqlen, stream);
+}
+
+extern "C" int evo_decode_qkv_prep_rows(void* qkv, void* cache, const void* cos, const void* sin, const int64_t* pos,
+                                        int B, int H, int hd, int64_t max_seqlen, void* stream) {
+  return decode_qkv_prep<true>("evo_decode_qkv_prep_rows", qkv, cache, cos, sin, pos, B, H, hd, max_seqlen, stream);
 }
 
 extern "C" size_t evo_decode_attn_workspace(int B, int H, int nsplit) { return (size_t)B * H * nsplit * (HD + 2) * sizeof(float); }
 
-extern "C" int evo_decode_attn(const void* qkv, const void* cache, void* out, const int64_t* pos, int B, int H, int hd,
-                               int64_t max_seqlen, int nsplit, float softmax_scale, void* workspace, size_t workspace_bytes, void* stream) {
-  EVO_REQUIRE(hd == HD, "evo_decode_attn: head_dim %d unsupported", hd);
-  EVO_REQUIRE(nsplit >= 1 && nsplit <= 64, "evo_decode_attn: bad nsplit %d", nsplit);
-  EVO_REQUIRE(workspace && workspace_bytes >= evo_decode_attn_workspace(B, H, nsplit), "evo_decode_attn: workspace too small");
+template <bool ROWS>
+static int decode_attn(const char* name, const void* qkv, const void* cache, void* out, const int64_t* pos, int B, int H, int hd,
+                       int64_t max_seqlen, int nsplit, float softmax_scale, void* workspace, size_t workspace_bytes, void* stream) {
+  EVO_REQUIRE(hd == HD, "%s: head_dim %d unsupported", name, hd);
+  EVO_REQUIRE(nsplit >= 1 && nsplit <= 64, "%s: bad nsplit %d", name, nsplit);
+  EVO_REQUIRE(workspace && workspace_bytes >= evo_decode_attn_workspace(B, H, nsplit), "%s: workspace too small", name);
   float* part_o = (float*)workspace;
   float* part_ml = part_o + (size_t)B * H * nsplit * HD;
   static const bool force_v1 = getenv("EVO_B200_DECODE_ATTN_V1") != nullptr;
@@ -302,20 +319,30 @@ extern "C" int evo_decode_attn(const void* qkv, const void* cache, void* out, co
     int rc = make_tmap_nd_bf16(&tm, cache, 3, dims, str, box, false);
     if (rc) return rc;
     static unsigned long long attr_done = 0;
-    if ((rc = ensure_dyn_smem(decode_attn_tma_kernel, ATT2_SMEM, attr_done))) return rc;
-    EVO_CUDA(launch_pdl(decode_attn_tma_kernel, dim3(H, B, nsplit), dim3(160), (size_t)ATT2_SMEM, (cudaStream_t)stream, tm, (const bf16*)qkv, part_o, part_ml,
+    if ((rc = ensure_dyn_smem(decode_attn_tma_kernel<ROWS>, ATT2_SMEM, attr_done))) return rc;
+    EVO_CUDA(launch_pdl(decode_attn_tma_kernel<ROWS>, dim3(H, B, nsplit), dim3(160), (size_t)ATT2_SMEM, (cudaStream_t)stream, tm, (const bf16*)qkv, part_o, part_ml,
                         (const long long*)pos, H, (long long)max_seqlen, nsplit, softmax_scale));
-    rc = check_launch("evo_decode_attn");
+    rc = check_launch(name);
     if (rc) return rc;
     EVO_CUDA(launch_pdl(decode_attn_merge_kernel, dim3(H, B), dim3(HD), 0, (cudaStream_t)stream, (const float*)part_o, (const float*)part_ml, (bf16*)out, H, nsplit));
     return check_launch("evo_decode_attn_merge");
   }
-  EVO_CUDA(launch_pdl(decode_attn_kernel, dim3(H, B, nsplit), dim3(DT), 0, (cudaStream_t)stream, (const bf16*)qkv, (const bf16*)cache, part_o, part_ml,
+  EVO_CUDA(launch_pdl(decode_attn_kernel<ROWS>, dim3(H, B, nsplit), dim3(DT), 0, (cudaStream_t)stream, (const bf16*)qkv, (const bf16*)cache, part_o, part_ml,
                       (const long long*)pos, H, max_seqlen, nsplit, softmax_scale));
-  int rc = check_launch("evo_decode_attn");
+  int rc = check_launch(name);
   if (rc) return rc;
   EVO_CUDA(launch_pdl(decode_attn_merge_kernel, dim3(H, B), dim3(HD), 0, (cudaStream_t)stream, (const float*)part_o, (const float*)part_ml, (bf16*)out, H, nsplit));
   return check_launch("evo_decode_attn_merge");
+}
+
+extern "C" int evo_decode_attn(const void* qkv, const void* cache, void* out, const int64_t* pos, int B, int H, int hd,
+                               int64_t max_seqlen, int nsplit, float softmax_scale, void* workspace, size_t workspace_bytes, void* stream) {
+  return decode_attn<false>("evo_decode_attn", qkv, cache, out, pos, B, H, hd, max_seqlen, nsplit, softmax_scale, workspace, workspace_bytes, stream);
+}
+
+extern "C" int evo_decode_attn_rows(const void* qkv, const void* cache, void* out, const int64_t* pos, int B, int H, int hd,
+                                    int64_t max_seqlen, int nsplit, float softmax_scale, void* workspace, size_t workspace_bytes, void* stream) {
+  return decode_attn<true>("evo_decode_attn_rows", qkv, cache, out, pos, B, H, hd, max_seqlen, nsplit, softmax_scale, workspace, workspace_bytes, stream);
 }
 
 extern "C" int evo_advance_position(int64_t* pos, int64_t delta, void* stream) {

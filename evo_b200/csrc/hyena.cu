@@ -191,19 +191,21 @@ __global__ void __launch_bounds__(THREADS) hyena_scan_kernel(const Args a) {
   }
 }
 
-// out = p^{total_len - nseg_full... } fold: carry over all segments' zero-start end states (+ state_in)
+// out = p^{total_len - nseg_full... } fold: carry over all segments' zero-start end states (+ state_in).
+// lengths (B) or NULL: row b's sequence ends at lengths[b] (ragged rows), so each segment contributes its effective length.
 __global__ void hyena_fold_states_kernel(const float* __restrict__ seg_states, const float* __restrict__ state_in,
                                          const float* __restrict__ poles, float* __restrict__ out,
-                                         int B, int D, int nseg, long long seg_len, long long L) {
+                                         int B, int D, int nseg, long long seg_len, long long L, const int* __restrict__ lengths) {
   int idx = blockIdx.x * blockDim.x + threadIdx.x;   // (b, ch, s)
   if (idx >= B * D * NS) return;
   int s = idx % NS, ch = (idx / NS) % D, b = idx / (NS * D);
+  if (lengths) L = min(L, (long long)max(lengths[b], 0));
   float2 pp = reinterpret_cast<const float2*>(poles)[(long long)ch * NS + s];
   Cplx p = {pp.x, pp.y};
   Cplx acc = {0.f, 0.f};
   if (state_in) { float2 v = reinterpret_cast<const float2*>(state_in)[idx]; acc = {v.x, v.y}; }
   for (int q = 0; q < nseg; ++q) {
-    long long len = min(seg_len, L - (long long)q * seg_len);
+    long long len = max(0LL, min(seg_len, L - (long long)q * seg_len));
     float2 e = reinterpret_cast<const float2*>(seg_states)[(((long long)b * nseg + q) * D + ch) * NS + s];
     Cplx c = cmul(cpow_int(p, len), acc);
     acc = {c.r + e.x, c.i + e.y};
@@ -211,14 +213,16 @@ __global__ void hyena_fold_states_kernel(const float* __restrict__ seg_states, c
   reinterpret_cast<float2*>(out)[idx] = make_float2(acc.r, acc.i);
 }
 
+// lengths (B) or NULL: the two rows before row b's own end (ragged rows); rows are still L apart in z
 __global__ void fir_state_kernel(const bf16* __restrict__ z, const bf16* __restrict__ halo, bf16* __restrict__ out,
-                                 int B, long long L, long long C3) {
+                                 int B, long long L, long long C3, const int* __restrict__ lengths) {
   long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // (b, c)
   if (idx >= (long long)B * C3) return;
   long long b = idx / C3, c = idx % C3;
+  const long long Lb = lengths ? min(L, (long long)max(lengths[b], 0)) : L;
 #pragma unroll
   for (int k = 0; k < 2; ++k) {
-    long long t = L - 2 + k;
+    long long t = Lb - 2 + k;
     bf16 v = __float2bfloat16_rn(0.f);
     if (t >= 0) v = z[(b * L + t) * C3 + c];
     else if (halo) v = halo[(b * 2 + (t + 2)) * C3 + c];
@@ -324,7 +328,8 @@ static void segment_geometry(const evo_hyena_params* p, int& nseg, long long& se
   nseg = (int)((p->L + seg_len - 1) / seg_len);
 }
 
-extern "C" int evo_hyena_fwd(const evo_hyena_params* p, void* workspace, size_t workspace_bytes, void* stream) {
+// lengths == NULL: evo_hyena_fwd; otherwise evo_hyena_fwd_ragged (mode-split TMA path only, checked by the caller)
+static int hyena_fwd_impl(const evo_hyena_params* p, const int* lengths, void* workspace, size_t workspace_bytes, void* stream) {
   EVO_REQUIRE(p->S == NS, "evo_hyena_fwd: state_size %d unsupported (kernel is specialised for %d)", p->S, NS);
   EVO_REQUIRE(p->nheads > 0 && p->D % p->nheads == 0, "evo_hyena_fwd: D %% nheads != 0");
   EVO_REQUIRE(p->B > 0 && p->B <= 65535, "evo_hyena_fwd: bad batch %d", p->B);
@@ -349,6 +354,7 @@ extern "C" int evo_hyena_fwd(const evo_hyena_params* p, void* workspace, size_t 
     a.fir_w = (const bf16*)p->fir_w; a.fir_b = (const bf16*)p->fir_b; a.Dskip = (const bf16*)p->Dskip;
     a.poles = p->poles; a.residues = p->residues; a.halo = (const bf16*)p->halo; a.state_in = p->state_in; a.state_out = p->state_out;
     a.seg_states = (float*)workspace; a.B = p->B; a.D = p->D; a.nseg = nseg; a.L = p->L; a.seg_len = seg_len;
+    a.lengths = lengths;
     static unsigned long long done_s = 0, done_o = 0;
     if ((rc = ensure_dyn_smem(hyena_scan_tma_kernel<true>, smem_bytes(STAGES), done_s))) return rc;
     if ((rc = ensure_dyn_smem(hyena_scan_tma_kernel<false>, smem_bytes(STAGES), done_o))) return rc;
@@ -362,6 +368,14 @@ extern "C" int evo_hyena_fwd(const evo_hyena_params* p, void* workspace, size_t 
     dim3 grid(p->D / CH_PER_CTA, p->B, nseg), block(variant == 1 ? evo_hy3::THREADS : evo_hy2::THREADS);
     auto k_state = variant == 1 ? evo_hy3::hyena_scan_ms_kernel<true> : hyena_scan_tma_kernel<true>;
     auto k_out = variant == 1 ? evo_hy3::hyena_scan_ms_kernel<false> : hyena_scan_tma_kernel<false>;
+    if (lengths) {
+      EVO_REQUIRE(variant == 1, "evo_hyena_fwd_ragged: only the mode-split scan (EVO_B200_HYENA_VARIANT=1) takes per-row lengths");
+      static unsigned long long done_rs = 0, done_ro = 0;
+      if ((rc = ensure_dyn_smem(evo_hy3::hyena_scan_ms_kernel<true, true>, smem_bytes(STAGES), done_rs))) return rc;
+      if ((rc = ensure_dyn_smem(evo_hy3::hyena_scan_ms_kernel<false, true>, smem_bytes(STAGES), done_ro))) return rc;
+      k_state = evo_hy3::hyena_scan_ms_kernel<true, true>;
+      k_out = evo_hy3::hyena_scan_ms_kernel<false, true>;
+    }
     // ring depth 4 (96 KB): two CTAs can co-reside and hide each other's latency when the grid exceeds the SM count.
     // An 8-deep ring for single-CTA-per-SM grids was measured and did not help (1.21 vs 1.06-1.13 ms at B=8, L=8193).
     a.nst = 4;
@@ -403,15 +417,30 @@ extern "C" int evo_hyena_fwd(const evo_hyena_params* p, void* workspace, size_t 
   }
   if (p->state_only) {
     int n = p->B * p->D * NS;
-    hyena_fold_states_kernel<<<(n + 255) / 256, 256, 0, st>>>((const float*)workspace, p->state_in, p->poles, p->state_out, p->B, p->D, nseg, seg_len, p->L);
+    hyena_fold_states_kernel<<<(n + 255) / 256, 256, 0, st>>>((const float*)workspace, p->state_in, p->poles, p->state_out, p->B, p->D, nseg, seg_len, p->L, lengths);
     if ((rc = check_launch("hyena_fold_states"))) return rc;
   }
   if (p->fir_state_out) {
     long long n = (long long)p->B * 3 * p->D;
-    fir_state_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const bf16*)p->z, (const bf16*)p->halo, (bf16*)p->fir_state_out, p->B, p->L, 3LL * p->D);
+    fir_state_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const bf16*)p->z, (const bf16*)p->halo, (bf16*)p->fir_state_out, p->B, p->L, 3LL * p->D, lengths);
     if ((rc = check_launch("fir_state"))) return rc;
   }
   return 0;
+}
+
+extern "C" int evo_hyena_fwd(const evo_hyena_params* p, void* workspace, size_t workspace_bytes, void* stream) {
+  return hyena_fwd_impl(p, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" size_t evo_hyena_fwd_ragged_workspace(const evo_hyena_params* p) { return evo_hyena_fwd_workspace(p); }
+
+extern "C" int evo_hyena_fwd_ragged(const evo_hyena_params* p, const int32_t* lengths_dev, void* workspace, size_t workspace_bytes, void* stream) {
+  EVO_REQUIRE(lengths_dev != nullptr, "evo_hyena_fwd_ragged: lengths is NULL");
+  EVO_REQUIRE(p->halo == nullptr && p->state_in == nullptr, "evo_hyena_fwd_ragged: halo / state_in (a continued prefill) are not supported with per-row lengths");
+  EVO_REQUIRE(!p->reuse_segment_states, "evo_hyena_fwd_ragged: reuse_segment_states is not supported with per-row lengths");
+  EVO_REQUIRE(p->nheads > 0 && p->D % p->nheads == 0 && use_tma_path(p),
+              "evo_hyena_fwd_ragged: needs head_dim 128 and D %% %d == 0 (the mode-split scan)", evo_hy2::CH_PER_CTA);
+  return hyena_fwd_impl(p, lengths_dev, workspace, workspace_bytes, stream);
 }
 
 extern "C" int evo_hyena_step(const void* u, void* y, void* fir_state, float* state,

@@ -45,7 +45,11 @@ __device__ __forceinline__ uint32_t mul_bf2(uint32_t a, uint32_t b) { uint32_t d
 __device__ __forceinline__ uint32_t add_bf2(uint32_t a, uint32_t b) { uint32_t d; asm("add.rn.bf16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b)); return d; }
 __device__ __forceinline__ uint32_t ldg32(const bf16* p) { return __ldg(reinterpret_cast<const unsigned int*>(p)); }
 
-template <bool STATE_ONLY>
+// RAGGED: row b holds a.lengths[b] valid tokens (right-padded to L): the scan of each segment stops at the row's length, a
+// segment wholly past it is empty, and the state after the row's last token is written by the segment that holds that token.
+// Every segment before that one is full, so the in-kernel carry fold needs no per-row length.  With every length == L the
+// RAGGED instantiation computes exactly what the uniform one does.
+template <bool STATE_ONLY, bool RAGGED = false>
 __global__ void __launch_bounds__(THREADS, 1)
 hyena_scan_ms_kernel(const __grid_constant__ CUtensorMap tmZ, const Args2 a) {
   extern __shared__ uint8_t smem_raw[];
@@ -56,9 +60,17 @@ hyena_scan_ms_kernel(const __grid_constant__ CUtensorMap tmZ, const Args2 a) {
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int cb = blockIdx.x, b = blockIdx.y, seg = blockIdx.z;
+  const long long Lb = RAGGED ? min(a.L, (long long)max(a.lengths[b], 0)) : a.L;
+  const int last_seg = RAGGED ? (Lb > 0 ? (int)((Lb - 1) / a.seg_len) : 0) : a.nseg - 1;
   const long long t0 = (long long)seg * a.seg_len;
-  const long long t1 = min(a.L, t0 + a.seg_len);
+  const long long t1 = min(Lb, t0 + a.seg_len);
   const int n_tiles = t1 > t0 ? (int)((t1 - t0 + T2 - 1) / T2) : 0;
+  if (RAGGED && n_tiles == 0 && (STATE_ONLY || seg != last_seg)) {
+    // nothing of this row here; the state pass still leaves a zero end state for the fold
+    if (STATE_ONLY && threadIdx.x < 256)
+      for (int i = threadIdx.x; i < CH_PER_CTA * NS * 2; i += 256) a.seg_states[(((long long)b * a.nseg + seg) * a.D + cb * CH_PER_CTA) * NS * 2 + i] = 0.f;
+    return;
+  }
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], CWARPS); }
@@ -256,7 +268,7 @@ hyena_scan_ms_kernel(const __grid_constant__ CUtensorMap tmZ, const Args2 a) {
 
   float* dst = nullptr;
   if (STATE_ONLY) dst = a.seg_states + ((((long long)b * a.nseg + seg) * a.D + ch) * NS) * 2;
-  else if (a.state_out && seg == a.nseg - 1) dst = a.state_out + (((long long)b * a.D + ch) * NS) * 2;
+  else if (a.state_out && seg == last_seg) dst = a.state_out + (((long long)b * a.D + ch) * NS) * 2;
   if (dst) {
     float2* e = reinterpret_cast<float2*>(dst) + m0;
 #pragma unroll

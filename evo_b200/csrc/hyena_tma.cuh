@@ -37,6 +37,7 @@ struct Args2 {
   float* seg_states;
   int B, D, nseg, nst;
   long long L, seg_len;
+  const int* lengths;          // (B) valid tokens per row (evo_hyena_fwd_ragged); NULL = every row has L
 };
 
 __device__ __forceinline__ float2 unpack2(uint32_t v) { return make_float2(bf_lo(v), bf_hi(v)); }

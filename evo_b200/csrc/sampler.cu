@@ -159,6 +159,44 @@ __global__ void __launch_bounds__(MAXV) sample_step_kernel(const bf16* __restric
   if (threadIdx.x == 0) x[row] = tok;
 }
 
+// one step of the ragged loop: row b has its own forced prefix and its own number of recorded tokens.  A row whose
+// steps are done (i >= n_forced[b] + n_out[b]) neither samples nor records, and keeps its input token.
+__global__ void __launch_bounds__(MAXV) sample_step_rows_kernel(const bf16* __restrict__ logits, long long* __restrict__ x, int V,
+                                                               const evo_ragged_loop_params* __restrict__ lp, const long long* __restrict__ step_dev) {
+  pdl_launch_dependents(); pdl_wait();
+  const int row = blockIdx.x;
+  const long long i = *step_dev;
+  const evo_ragged_loop_params P = *lp;
+  const long long nf = P.n_forced[row], no = P.n_out[row];
+  long long tok;
+  if (i < nf) {
+    tok = P.forced[(long long)row * P.forced_stride + i];
+  } else {
+    const long long k = i - nf;
+    if (k >= no) return;                                             // uniform per CTA
+    const SampleCfg cfg = {P.top_k, P.top_p, P.temperature, (unsigned long long)P.seed};
+    tok = sample_row(logits + (long long)row * V, V, cfg, (uint64_t)i, row);
+    const long long col = P.out_cols - no + k;                        // the row's tokens fill its last n_out columns
+    if (threadIdx.x == 0 && P.picked) P.picked[(long long)row * P.out_cols + col] = tok;
+    if (P.kept_logits && threadIdx.x < V)
+      P.kept_logits[((long long)row * P.out_cols + col) * V + threadIdx.x] = __bfloat162float(logits[(long long)row * V + threadIdx.x]);
+  }
+  if (threadIdx.x == 0) x[row] = tok;
+}
+
+// step += 1; pos[b] = start[b] + min(step, steps_b - 1): a finished row stays at the position of its last step
+__global__ void ragged_advance_kernel(long long* __restrict__ pos, long long* __restrict__ step, const evo_ragged_loop_params* __restrict__ lp, int B) {
+  pdl_launch_dependents(); pdl_wait();
+  const long long s = *step + 1;
+  __syncthreads();                                                    // every thread has read the old step
+  const int b = threadIdx.x;
+  if (b < B) {
+    const long long steps = lp->n_forced[b] + lp->n_out[b];
+    pos[b] = lp->start[b] + max(0LL, min(s, steps - 1));
+  }
+  if (b == 0) *step = s;
+}
+
 __global__ void advance2_kernel(long long* a, long long* b, long long delta) {
   pdl_launch_dependents(); pdl_wait();
   if (threadIdx.x == 0) { if (a) *a += delta; if (b) *b += delta; }
@@ -184,6 +222,23 @@ extern "C" int evo_sample_step(const void* logits, int64_t* x, int B, int V, con
   EVO_CUDA(launch_pdl(sample_step_kernel, dim3(B), dim3((V + 31) / 32 * 32), 0, (cudaStream_t)stream, (const bf16*)logits, (long long*)x, V,
                       loop_params_dev, (const long long*)step_dev));
   return check_launch("evo_sample_step");
+}
+
+extern "C" int evo_sample_step_rows(const void* logits, int64_t* x, int B, int V, const evo_ragged_loop_params* loop_params_dev,
+                                    const int64_t* step_dev, void* stream) {
+  EVO_REQUIRE(V > 0 && V <= MAXV, "evo_sample_step_rows: vocabulary %d unsupported (<= %d)", V, MAXV);
+  EVO_REQUIRE(B >= 0 && B <= 65535, "evo_sample_step_rows: bad batch %d", B);
+  if (B == 0) return 0;
+  EVO_CUDA(launch_pdl(sample_step_rows_kernel, dim3(B), dim3((V + 31) / 32 * 32), 0, (cudaStream_t)stream, (const bf16*)logits, (long long*)x, V,
+                      loop_params_dev, (const long long*)step_dev));
+  return check_launch("evo_sample_step_rows");
+}
+
+extern "C" int evo_ragged_advance(int64_t* pos, int64_t* step, const evo_ragged_loop_params* loop_params_dev, int B, void* stream) {
+  EVO_REQUIRE(B >= 1 && B <= 1024, "evo_ragged_advance: batch %d unsupported (1..1024)", B);
+  EVO_CUDA(launch_pdl(ragged_advance_kernel, dim3(1), dim3((B + 31) / 32 * 32), 0, (cudaStream_t)stream, (long long*)pos, (long long*)step,
+                      loop_params_dev, B));
+  return check_launch("evo_ragged_advance");
 }
 
 extern "C" int evo_advance_counters(int64_t* a, int64_t* b, int64_t delta, void* stream) {

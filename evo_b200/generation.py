@@ -15,7 +15,7 @@ from __future__ import annotations
 
 import os
 import sys
-from typing import List, Optional, Tuple
+from typing import List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -27,6 +27,35 @@ from .tokenizer import CharLevelTokenizer
 
 def _gb(device) -> float:
     return torch.cuda.memory_allocated(device=device) / 1e9 if torch.cuda.is_available() else 0.0
+
+
+# rows per batch of the ragged path: the stream-K decode GEMM takes at most 64 rows
+RAGGED_CHUNK = 64
+
+
+class RowSchedule(NamedTuple):
+    prefill: int     # P_b = min(force_prompt_threshold, len_b): tokens of the parallel prefill
+    start: int       # position of loop step 0: the FULL prompt length, even after a truncated prefill (Q1)
+    n_forced: int    # prompt tokens teacher-forced inside the loop (the tail after its first token)
+    n_out: int       # tokens sampled inside the loop (n_tokens - 1 when the prefill logits give the first one)
+    steps: int       # single-token steps the loop runs = n_forced + n_out
+
+
+def ragged_schedule(lengths: Sequence[int], threshold: int, n_tokens: int) -> List[RowSchedule]:
+    """The cached generation protocol of each prompt, as the device loop runs it (evo/generation.py:131-189): prefill the
+    first P = min(threshold, len) tokens in parallel; if the prompt has a tail past P, the prefill's logits are dropped,
+    loop step 0 feeds tail[0] at position len (Q1: positions P..len-1 are skipped) and the rest of the tail is forced
+    before n_tokens tokens are sampled; otherwise the prefill's logits give the first token and the loop samples the
+    other n_tokens - 1, starting at position len.  Step i of a row runs at position start + i."""
+    out = []
+    for n in lengths:
+        n = int(n)
+        prefill = min(int(threshold), n)
+        tail = n - prefill
+        n_forced = max(tail - 1, 0)
+        n_out = int(n_tokens) if tail else max(int(n_tokens) - 1, 0)
+        out.append(RowSchedule(prefill, n, n_forced, n_out, n_forced + n_out))
+    return out
 
 
 class Generator:
@@ -78,6 +107,7 @@ class Generator:
         n_seq, n_tail = window.shape[0], tail.shape[1]
         dev = window.device
         total = n_tail + num_tokens
+        plan = ragged_schedule([window.shape[1]], x.shape[1], num_tokens)[0]     # the same bookkeeping as the ragged path
         picked = torch.empty(n_seq, num_tokens, dtype=torch.long, device=dev)
         kept_logits = torch.empty(n_seq, num_tokens, tk.vocab_size, dtype=torch.float, device=dev)
         pick_args = dict(top_k=self.top_k, top_p=self.top_p, temperature=self.temperature)
@@ -98,10 +128,10 @@ class Generator:
                 kept_logits[:, 0], picked[:, 0] = head, token
                 first = 1
             start = full_prompt.shape[-1]                      # the reference's jump to the full prompt length (Q1)
-            forced, n_loop = tail[:, 1:], total - 1
+            forced, n_loop = tail[:, 1:], plan.steps
         if n_loop > 0:
             got, got_logits = self.model.decode_loop(token, state, n_loop, start, forced=forced if forced.shape[1] else None,
-                                                     n_out=num_tokens - first, **pick_args)
+                                                     n_out=plan.n_out if not resumed else num_tokens - first, **pick_args)
             picked[:, first:], kept_logits[:, first:] = got, got_logits
         if stop_at_eos and num_tokens >= 2 and bool((picked[0, -2:] == tk.eos).all()):
             print("Stopping generation at EOS")              # report only, as in the reference (Q2)
@@ -124,6 +154,56 @@ class Generator:
         _lib.check(_lib.lib().evo_sample(_lib.ptr(head), _lib.ptr(out), head.shape[0], head.shape[1], int(self.top_k), float(self.top_p), float(self.temperature),
                                          seed, 0, C.c_void_p(torch.cuda.current_stream(head.device).cuda_stream)), "evo_sample")
         return out
+
+    def can_run_ragged(self, device, cached_generation: bool) -> bool:
+        """Whether generate_ragged applies: cached generation with the loop on a CUDA device (model.decode_loop_ragged)."""
+        return (bool(cached_generation) and self.device_loop and hasattr(self.model, "decode_loop_ragged")
+                and torch.device(device).type == "cuda")
+
+    def generate_ragged(self, device: str, prompts_ids: Sequence[torch.Tensor], num_tokens: int = 32, force_prompt_threshold: int = 128,
+                        seed: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Prompts of different lengths as ONE batch through the on-device loop.  Row b produces what generate() produces for
+        prompts_ids[b] alone with cached generation (same prefill slice, same teacher-forced tail, Q1's position jump, same
+        token/logit alignment), up to the rounding of a different batch shape.  prompts_ids: 1-D (or (1, n)) id tensors,
+        at most 64.  Returns (picked (B, num_tokens) int64, kept_logits (B, num_tokens, V) fp32); there is no resumable
+        state, since the rows end at different positions."""
+        from ._lib import EvoError
+        rows = [torch.as_tensor(p).reshape(-1).to(device=device, dtype=torch.long) for p in prompts_ids]
+        B, num_tokens = len(rows), int(num_tokens)
+        if not 1 <= B <= RAGGED_CHUNK:
+            raise ValueError(f"generate_ragged takes 1..{RAGGED_CHUNK} prompts, got {B}")
+        if min(r.numel() for r in rows) < 1 or num_tokens < 1:
+            raise ValueError("every prompt needs a token and num_tokens must be >= 1")
+        plan = ragged_schedule([r.numel() for r in rows], force_prompt_threshold, num_tokens)
+        W = max(s.prefill for s in plan)
+        F = max(s.n_forced for s in plan)
+        ids = torch.zeros(B, W, dtype=torch.long, device=device)
+        forced = torch.zeros(B, max(F, 1), dtype=torch.long, device=device)
+        tail0 = torch.zeros(B, dtype=torch.long, device=device)
+        for b, (r, s) in enumerate(zip(rows, plan)):
+            ids[b, :s.prefill] = r[:s.prefill]
+            if r.numel() > s.prefill:
+                tail0[b] = r[s.prefill]
+                forced[b, :s.n_forced] = r[s.prefill + 1:]
+        has_tail = torch.tensor([r.numel() > s.prefill for r, s in zip(rows, plan)], device=device)
+        state = self.model.initialize_inference_params()
+        for holder in (state["mha"], state["hyena"]):
+            holder.max_batch_size = B
+        cap = state["mha"].max_seqlen
+        for b, s in enumerate(plan):                           # checked per row, before anything runs (mha.py:367)
+            if s.start + s.steps > cap:
+                raise EvoError(f"row {b}: sequence length {s.start + s.steps} exceeds the KV cache ({cap}) (mha.py:367)")
+        with torch.inference_mode():
+            head = self.model.prefill_ragged(ids, [s.prefill for s in plan], state)
+        sampled = self._pick_device(head)
+        token = torch.where(has_tail, tail0, sampled)
+        pick_args = dict(top_k=self.top_k, top_p=self.top_p, temperature=self.temperature)
+        picked, kept = self.model.decode_loop_ragged(token, state, [s.start for s in plan], [s.n_forced for s in plan], [s.n_out for s in plan],
+                                                     forced=forced if F else None, out_cols=num_tokens, seed=seed, **pick_args)
+        first = ~has_tail                                      # rows whose first token came from the prefill's logits
+        picked[first, 0] = sampled[first]
+        kept[first, 0] = head[first].float()
+        return picked, kept
 
     # -- public ---------------------------------------------------------------------------
     def generate(self, device: str, input_string: str = None, input_ids: torch.Tensor = None, num_tokens: int = 32,
@@ -186,12 +266,17 @@ class Generator:
 def generate(prompt_seqs: List[str], model, tokenizer: CharLevelTokenizer, n_tokens: int = 100, temperature: float = 0.0,
              top_k: int = 1, top_p: float = 1.0, batched: bool = True, prepend_bos: bool = False,
              cached_generation: bool = False, force_prompt_threshold: int = 128, verbose: int = 1,
-             device: str = "cuda:0", **kwargs) -> Tuple[List[str], List[float]]:
+             device: str = "cuda:0", ragged: bool = False, **kwargs) -> Tuple[List[str], List[float]]:
     """Sequences and mean log-likelihood "scores" for a list of prompts.  Prompts of one common
-    length run as one batch; anything else falls back to one prompt at a time (with a note on stderr)."""
+    length run as one batch; anything else falls back to one prompt at a time (with a note on stderr).
+    ragged=True: prompts of different lengths run as batches of up to 64 through the on-device loop
+    (Generator.generate_ragged); each row produces what its prompt produces alone.  It applies to cached generation
+    with the loop on a CUDA device; otherwise generate() behaves as without it."""
     model.eval()
     engine = Generator(model, tokenizer, top_k=top_k, top_p=top_p, temperature=temperature)
     uniform = len({len(p) for p in prompt_seqs}) <= 1
+    if ragged and batched and not uniform and engine.can_run_ragged(device, cached_generation):
+        return _generate_ragged(engine, prompt_seqs, tokenizer, n_tokens, prepend_bos, force_prompt_threshold, verbose, device)
     if batched and uniform:
         work = [list(prompt_seqs)]
     else:
@@ -219,6 +304,28 @@ def generate(prompt_seqs: List[str], model, tokenizer: CharLevelTokenizer, n_tok
         per_token = logits_to_logprobs(new_logits, new_ids).float().cpu().numpy()
         scores.extend(float(np.mean(row)) for row in per_token)
 
+    if verbose:
+        for prompt, text, score in zip(prompt_seqs, texts, scores):
+            print(f'Prompt: "{prompt}",\tOutput: "{text}",\tScore: {score}')
+    return texts, scores
+
+
+def _generate_ragged(engine: Generator, prompt_seqs: List[str], tokenizer: CharLevelTokenizer, n_tokens: int, prepend_bos: bool,
+                     force_prompt_threshold: int, verbose: int, device: str) -> Tuple[List[str], List[float]]:
+    """generate(ragged=True): prompts sorted by length, cut into batches of at most RAGGED_CHUNK rows, results back in
+    input order.  Texts and scores are computed per row exactly as for a batch of one."""
+    ids = [prepare_batch([p], tokenizer, prepend_bos=prepend_bos, device=device)[0][0] for p in prompt_seqs]
+    order = sorted(range(len(ids)), key=lambda i: ids[i].numel())
+    texts: List[Optional[str]] = [None] * len(ids)
+    scores: List[Optional[float]] = [None] * len(ids)
+    for c in range(0, len(order), RAGGED_CHUNK):
+        chunk = order[c:c + RAGGED_CHUNK]
+        new_ids, new_logits = engine.generate_ragged(device, [ids[i] for i in chunk], num_tokens=n_tokens, force_prompt_threshold=force_prompt_threshold)
+        decoded = tokenizer.detokenize_batch(new_ids)
+        for r, i in enumerate(chunk):
+            texts[i] = decoded[r]
+            # logits_to_logprobs(trim_bos=True) pairs logits[i] with token[i+1]: the reference's alignment (Q3)
+            scores[i] = float(np.mean(logits_to_logprobs(new_logits[r:r + 1], new_ids[r:r + 1]).float().cpu().numpy()[0]))
     if verbose:
         for prompt, text, score in zip(prompt_seqs, texts, scores):
             print(f'Prompt: "{prompt}",\tOutput: "{text}",\tScore: {score}')

@@ -234,6 +234,7 @@ class StripedHyena(nn.Module):
         self._tiled = None   # tile-major weight copies for the weight-streaming decode GEMMs
         self._decode = None  # cached CUDA graph of one decode step (see _decode_forward)
         self._loop = None    # cached CUDA graph of one step of the on-device generation loop (see decode_loop)
+        self._loop_ragged = None   # the same for prompts of different lengths (see decode_loop_ragged)
         self._prof = None   # set to a list to record (kind, algorithmic work, start event, end event) per kernel call
 
     # ---- reference API ------------------------------------------------------------------
@@ -257,6 +258,7 @@ class StripedHyena(nn.Module):
         self._packed = None
         self._decode = None
         self._loop = None
+        self._loop_ragged = None
         self._tiled = None
         return out
 
@@ -266,6 +268,7 @@ class StripedHyena(nn.Module):
         self._rope = None
         self._decode = None
         self._loop = None
+        self._loop_ragged = None
         self._tiled = None
         return out
 
@@ -384,7 +387,7 @@ class StripedHyena(nn.Module):
         self._gemm(g, pk["w3"], out, M, d, pk["ipad"], EPI_RESID, resid=u)
         return out
 
-    def _hyena_block(self, i, blk, u, B, L, ip: Optional[RecurrentInferenceParams]):
+    def _hyena_block(self, i, blk, u, B, L, ip: Optional[RecurrentInferenceParams], lengths=None):
         cfg = self.config
         d, H = cfg.hidden_size, cfg.num_attention_heads
         M = B * L
@@ -421,9 +424,14 @@ class StripedHyena(nn.Module):
                 st_out = torch.empty(B, d, cfg.state_size, 2, dtype=torch.float32, device=dev)
                 fs_out = torch.empty(B, 3 * d, 2, dtype=torch.bfloat16, device=dev)
                 hp.state_out, hp.fir_state_out = st_out.data_ptr(), fs_out.data_ptr()
-            ws_bytes = lib.evo_hyena_fwd_workspace(C.byref(hp))
-            ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
-            self._record("hyena", 8.0 * B * L * d, lambda: check(lib.evo_hyena_fwd(C.byref(hp), ptr(ws), ws_bytes, self._stream()), "evo_hyena_fwd"))
+            if lengths is not None:     # right-padded rows (prefill_ragged): each row's scan and states end at its own length
+                ws_bytes = lib.evo_hyena_fwd_ragged_workspace(C.byref(hp))
+                ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+                self._record("hyena", 8.0 * B * L * d, lambda: check(lib.evo_hyena_fwd_ragged(C.byref(hp), ptr(lengths), ptr(ws), ws_bytes, self._stream()), "evo_hyena_fwd_ragged"))
+            else:
+                ws_bytes = lib.evo_hyena_fwd_workspace(C.byref(hp))
+                ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+                self._record("hyena", 8.0 * B * L * d, lambda: check(lib.evo_hyena_fwd(C.byref(hp), ptr(ws), ws_bytes, self._stream()), "evo_hyena_fwd"))
             if ip is not None:
                 ip.state_dict[i] = torch.view_as_complex(st_out)
                 ip.fir_state_dict[i] = fs_out
@@ -502,8 +510,9 @@ class StripedHyena(nn.Module):
             self._gemm(u, self.unembed.weight, logits, M, V, d, EPI_NONE)
         return logits.view(B, L, V), inference_params_dict
 
-    def _backbone(self, x, B, L, inference_params_dict=None):
-        """embed -> all blocks -> final norm: the (B*L, D) bf16 input of the unembedding."""
+    def _backbone(self, x, B, L, inference_params_dict=None, lengths=None):
+        """embed -> all blocks -> final norm: the (B*L, D) bf16 input of the unembedding.
+        lengths: (B) int32 on the device for right-padded rows (see prefill_ragged), else None."""
         M, d, V = B * L, self.config.hidden_size, self.config.vocab_size
         dev = x.device
         u = torch.empty(M, d, dtype=torch.bfloat16, device=dev)
@@ -515,12 +524,54 @@ class StripedHyena(nn.Module):
                 u = self._attention_block(i, blk, u, B, L, ip)
             else:
                 ip = inference_params_dict["hyena"] if inference_params_dict is not None else None
-                u = self._hyena_block(i, blk, u, B, L, ip)
+                u = self._hyena_block(i, blk, u, B, L, ip, lengths)
         if self.norm is not None:
             xn = torch.empty_like(u)
             self._rmsnorm(u, self.norm.scale, xn, M)
             u = xn
         return u
+
+    def prefill_ragged(self, ids, lengths, ipd):
+        """Prefill of prompts of different lengths in one batch: ids (B, W) right-padded, row b's prompt is ids[b, :lengths[b]].
+        Populates the fresh inference params `ipd` as B separate prefills would -- Hyena state and FIR state after each row's
+        own last token (evo_hyena_fwd_ragged), keys and values of positions [0, lengths[b]) in the KV cache -- and returns the
+        (B, V) bf16 logits at each row's last prompt position.  Positions past a row's length are computed and discarded:
+        attention is causal, so they never reach a valid position, and their KV slots are overwritten by the row's decode
+        steps before any step reads them.  Only the B rows the caller needs go through the unembedding."""
+        if ids.dim() != 2 or ids.dtype not in (torch.int32, torch.int64):
+            raise TypeError("input ids must be (batch, length) int32/int64")
+        self._ensure_packed()
+        dev = self.embedding_layer.weight.device
+        if ids.device != dev:
+            raise _lib.EvoError(f"input ids on {ids.device}, model on {dev}")
+        B, W = ids.shape
+        lens = [int(n) for n in lengths]
+        if len(lens) != B or (B and (min(lens) < 1 or max(lens) > W)):
+            raise ValueError(f"lengths must be {B} values in [1, {W}], got {lens}")
+        mha_ip, hy_ip = ipd["mha"], ipd["hyena"]
+        if mha_ip.seqlen_offset or hy_ip.seqlen_offset or mha_ip.key_value_memory_dict or hy_ip.state_dict or hy_ip.fir_state_dict:
+            raise _lib.EvoError("prefill_ragged needs fresh inference params (initialize_inference_params())")
+        d, V = self.config.hidden_size, self.config.vocab_size
+        x = ids.contiguous()
+        with torch.cuda.device(dev), torch.no_grad():
+            prev = self._loop_ragged
+            if prev is not None:
+                # the KV caches the ragged loop's captured step was recorded with: zeroed (what a fresh cache holds) and reused,
+                # so a second call of the same shape replays that step instead of capturing a new one
+                H = self.config.num_attention_heads
+                want = (mha_ip.max_batch_size, mha_ip.max_seqlen, 2, H, d // H)
+                with torch.inference_mode():
+                    for i, c in prev["kv"].items():
+                        if tuple(c.shape) == want:
+                            mha_ip.key_value_memory_dict[i] = c.zero_()
+            lens_dev = torch.tensor(lens, dtype=torch.int32, device=dev)
+            u = self._backbone(x, B, W, ipd, lengths=lens_dev)
+            last = torch.tensor([b * W + n - 1 for b, n in enumerate(lens)], dtype=torch.int64, device=dev)
+            rows = torch.empty(B, d, dtype=torch.bfloat16, device=dev)
+            check(_lib.lib().evo_embed(ptr(last), 1, ptr(u), ptr(rows), B, d, B * W, self._stream()), "evo_embed")   # row gather
+            logits = torch.empty(B, V, dtype=torch.bfloat16, device=dev)
+            self._gemm(rows, self.unembed.weight, logits, B, V, d, EPI_NONE)
+        return logits
 
     def score_tokens(self, input_ids, want_logprobs=True, want_entropy=False):
         """Fused scoring head (SURVEY 8f-1): what evo/scoring.py computes from `model(input_ids)` -- log_softmax of the
@@ -587,16 +638,17 @@ class StripedHyena(nn.Module):
         self._tiled = t
         return t
 
-    def _decode_body(self, x, pos_dev, ipd, B):
-        """One token per sequence through all blocks; every launch reads the position from pos_dev."""
+    def _decode_body(self, x, pos_dev, ipd, B, rows=False):
+        """One token per sequence through all blocks; every launch reads the position from pos_dev.
+        rows: pos_dev is a (B) vector, one position per row (the *_rows attention kernels); else one (1) position."""
         lib = _lib.lib()
         prev = lib.evo_set_pdl(int(self.decode_pdl))
         try:
-            return self._decode_body_impl(x, pos_dev, ipd, B)
+            return self._decode_body_impl(x, pos_dev, ipd, B, rows)
         finally:
             lib.evo_set_pdl(prev)
 
-    def _decode_body_impl(self, x, pos_dev, ipd, B):
+    def _decode_body_impl(self, x, pos_dev, ipd, B, rows=False):
         cfg = self.config
         d, H, V = cfg.hidden_size, cfg.num_attention_heads, cfg.vocab_size
         hd = d // H
@@ -614,6 +666,7 @@ class StripedHyena(nn.Module):
             else:
                 self._gemm(a, w, out, B, N, K, epi, bias=bias, resid=resid, variant=G2)
 
+        qkv_prep, attn = (lib.evo_decode_qkv_prep_rows, lib.evo_decode_attn_rows) if rows else (lib.evo_decode_qkv_prep, lib.evo_decode_attn)
         u = torch.empty(B, d, dtype=torch.bfloat16, device=dev)
         check(lib.evo_embed(ptr(x), int(x.dtype == torch.int64), ptr(self.embedding_layer.weight), ptr(u), B, d, V, self._stream()), "evo_embed")
         nsplit = max(1, min(16, -(-8 * torch.cuda.get_device_properties(dev).multi_processor_count // (H * B))))   # >= ~4 waves of 2 CTAs/SM
@@ -627,11 +680,11 @@ class StripedHyena(nn.Module):
                 lin(xn, wsel(i, "in", mha.Wqkv.weight), qkv, 3 * d, d, EPI_BIAS if mha.Wqkv.bias is not None else EPI_NONE, bias=mha.Wqkv.bias)
                 cache = mha_ip.key_value_memory_dict[i]
                 cos, sin = self._rope_tables(cache.shape[1], dev)
-                check(lib.evo_decode_qkv_prep(ptr(qkv), ptr(cache), ptr(cos), ptr(sin), ptr(pos_dev), B, H, hd, cache.shape[1], self._stream()), "evo_decode_qkv_prep")
+                check(qkv_prep(ptr(qkv), ptr(cache), ptr(cos), ptr(sin), ptr(pos_dev), B, H, hd, cache.shape[1], self._stream()), "evo_decode_qkv_prep")
                 nws = lib.evo_decode_attn_workspace(B, H, nsplit)
                 ws = torch.empty(nws, dtype=torch.uint8, device=dev)
                 ctx = xn
-                check(lib.evo_decode_attn(ptr(qkv), ptr(cache), ptr(ctx), ptr(pos_dev), B, H, hd, cache.shape[1], nsplit,
+                check(attn(ptr(qkv), ptr(cache), ptr(ctx), ptr(pos_dev), B, H, hd, cache.shape[1], nsplit,
                                           1.0 / math.sqrt(hd), ptr(ws), nws, self._stream()), "evo_decode_attn")
                 lin(ctx, wsel(i, "out", mha.out_proj.weight), u2, d, d, EPI_BIAS_RESID if mha.out_proj.bias is not None else EPI_RESID,
                     bias=mha.out_proj.bias, resid=u)
@@ -759,6 +812,122 @@ class StripedHyena(nn.Module):
             mha_ip.seqlen_offset = hy_ip.seqlen_offset = end
             # the captured graph and its buffers stay alive in self._loop; the outputs are this call's own tensors
             return picked[:, :n_out], kept[:, :n_out]
+
+    def decode_loop_ragged(self, first_token, ipd, start, n_forced, n_out, *, forced=None, out_cols=None, top_k=1, top_p=0.0,
+                           temperature=1.0, seed=None):
+        """decode_loop for rows that sit at different positions (prompts of different lengths, after prefill_ragged).
+
+        Row b starts at position start[b], feeds first_token[b] at step 0, is teacher-forced with forced[b, :n_forced[b]],
+        then samples n_out[b] tokens; it runs n_forced[b] + n_out[b] steps and then stands still (keeps its position,
+        records nothing) while the longer rows finish.  Returns (picked (B, out_cols) int64, kept_logits (B, out_cols, V)
+        fp32): row b's tokens fill its LAST n_out[b] columns; columns before those are not written.
+        One CUDA graph per step, like decode_loop, with its own graph cache.  The cache keeps the state tensors the step was
+        captured with (the KV caches included) until the model is moved or reloaded; prefill_ragged and the next call of the
+        same shape reuse them, so that call replays the captured step.  The state holders' seqlen_offset are left as they
+        are: the rows end at different positions, so the state is not resumable through them."""
+        lib = _lib.lib()
+        dev = self.embedding_layer.weight.device
+        x = first_token.reshape(-1, 1).contiguous()
+        B = x.shape[0]
+        V = self.config.vocab_size
+        start, n_forced, n_out = ([int(v) for v in a] for a in (start, n_forced, n_out))
+        if not (len(start) == len(n_forced) == len(n_out) == B):
+            raise ValueError("start, n_forced and n_out need one entry per row")
+        if B > 64:
+            raise _lib.EvoError(f"decode_loop_ragged: batch {B} > 64 (the stream-K decode GEMM's limit)")
+        if min(n_forced + n_out) < 0:
+            raise ValueError("negative step counts")
+        out_cols = max(n_out) if out_cols is None else int(out_cols)
+        if max(n_out) > out_cols:
+            raise ValueError("n_out exceeds out_cols")
+        F = max(n_forced)
+        if F and (forced is None or forced.shape[0] != B or forced.shape[1] < F):
+            raise ValueError(f"forced must be (B, >= {F})")
+        if not self._can_step(ipd, B):
+            raise _lib.EvoError("decode_loop_ragged needs populated inference params (run prefill_ragged first)")
+        mha_ip, hy_ip = ipd["mha"], ipd["hyena"]
+        steps = [f + o for f, o in zip(n_forced, n_out)]
+        for i in mha_ip.key_value_memory_dict:
+            cap = mha_ip.key_value_memory_dict[i].shape[1]
+            for b in range(B):
+                if start[b] + steps[b] > cap:
+                    raise _lib.EvoError(f"row {b}: sequence length {start[b] + steps[b]} exceeds the KV cache ({cap}) (mha.py:367)")
+        n_steps = max(steps)
+        with torch.cuda.device(dev), torch.no_grad():
+            picked = torch.empty(B, max(out_cols, 1), dtype=torch.long, device=dev)
+            kept = torch.empty(B, max(out_cols, 1), V, dtype=torch.float32, device=dev)
+            if n_steps == 0:
+                return picked[:, :out_cols], kept[:, :out_cols]
+            self._ensure_packed()
+            for i in list(hy_ip.state_dict):
+                hy_ip.state_dict[i] = hy_ip.state_dict[i].contiguous()
+                hy_ip.fir_state_dict[i] = hy_ip.fir_state_dict[i].contiguous()
+            prev = self._loop_ragged
+            if prev is not None:
+                # move the Hyena states into the tensors the captured step was recorded with (a few MB per layer)
+                # (inference mode: the held tensors were made by a prefill under torch.inference_mode, as generate() runs it)
+                with torch.inference_mode():
+                    for store, held in ((hy_ip.state_dict, prev["hy"]), (hy_ip.fir_state_dict, prev["fir"])):
+                        for i, t in held.items():
+                            if i in store and store[i].shape == t.shape and store[i].dtype == t.dtype and store[i].data_ptr() != t.data_ptr():
+                                store[i] = t.copy_(store[i])
+            per_row = torch.tensor([n_forced, n_out, start], dtype=torch.int64, device=dev)
+            forced_c = forced[:, :F].to(dev, torch.long).contiguous() if F else None
+            if seed is None:
+                seed = int(torch.randint(0, 2 ** 62, (1,)).item())          # torch.manual_seed() governs reproducibility
+            lp = _lib.RaggedLoopParams(n_forced=per_row[0].data_ptr(), n_out=per_row[1].data_ptr(), start=per_row[2].data_ptr(),
+                                       forced=forced_c.data_ptr() if F else None, forced_stride=F,
+                                       picked=picked.data_ptr(), kept_logits=kept.data_ptr(), out_cols=picked.shape[1],
+                                       top_k=int(top_k), top_p=float(top_p), temperature=float(temperature), seed=seed)
+            key = ("ragged", B, tuple(hy_ip.state_dict[i].data_ptr() for i in sorted(hy_ip.state_dict)),
+                   tuple(hy_ip.fir_state_dict[i].data_ptr() for i in sorted(hy_ip.fir_state_dict)),
+                   tuple((mha_ip.key_value_memory_dict[i].data_ptr(), mha_ip.key_value_memory_dict[i].shape[1]) for i in sorted(mha_ip.key_value_memory_dict)))
+            st = self._loop_ragged
+            if st is None or st["key"] != key:
+                st = {"key": key, "graph": None, "x": torch.empty(B, 1, dtype=torch.long, device=dev), "pos": torch.zeros(B, dtype=torch.int64, device=dev),
+                      "step": torch.zeros(1, dtype=torch.int64, device=dev), "lp": torch.zeros(C.sizeof(_lib.RaggedLoopParams), dtype=torch.uint8, device=dev),
+                      "lp_host": torch.zeros(C.sizeof(_lib.RaggedLoopParams), dtype=torch.uint8).pin_memory(),
+                      # the state tensors the step is captured with stay alive here, so the next call can reuse them
+                      "hy": dict(hy_ip.state_dict), "fir": dict(hy_ip.fir_state_dict), "kv": dict(mha_ip.key_value_memory_dict)}
+                self._loop_ragged = st
+            if st.get("lp_copied") is not None:
+                st["lp_copied"].synchronize()       # a previous call's async copy may not have left the pinned staging buffer yet
+            C.memmove(st["lp_host"].data_ptr(), C.addressof(lp), C.sizeof(lp))
+            st["lp"].copy_(st["lp_host"], non_blocking=True)
+            st["lp_copied"] = torch.cuda.Event()
+            st["lp_copied"].record()
+            st["pos"].copy_(per_row[2])
+            st["step"].zero_()
+            st["x"].copy_(x.to(torch.long))
+
+            def one_step():
+                logits = self._decode_body(st["x"], st["pos"], ipd, B, rows=True)
+                prev = lib.evo_set_pdl(int(self.decode_pdl))
+                try:
+                    check(lib.evo_sample_step_rows(ptr(logits), ptr(st["x"]), B, V, ptr(st["lp"]), ptr(st["step"]), self._stream()), "evo_sample_step_rows")
+                    check(lib.evo_ragged_advance(ptr(st["pos"]), ptr(st["step"]), ptr(st["lp"]), B, self._stream()), "evo_ragged_advance")
+                finally:
+                    lib.evo_set_pdl(prev)
+
+            done = 0
+            if st["graph"] is None or st.get("ptrs") != self._graph_ptrs():
+                one_step()                      # eager step: allocates rope tables / workspaces the capture must not
+                done = 1
+                if self.decode_graph and n_steps > 1:
+                    g = torch.cuda.CUDAGraph()
+                    torch.cuda.synchronize()
+                    n0 = lib.evo_launch_count()
+                    with torch.cuda.graph(g):
+                        one_step()
+                    st["graph"], st["launches"], st["ptrs"] = g, lib.evo_launch_count() - n0, self._graph_ptrs()
+                    lib.evo_note_graph_replay(-st["launches"])
+            for _ in range(done, n_steps):
+                if st["graph"] is not None:
+                    st["graph"].replay()
+                    lib.evo_note_graph_replay(st["launches"])
+                else:
+                    one_step()
+            return picked[:, :out_cols], kept[:, :out_cols]
 
     def _graph_ptrs(self):
         """Addresses a captured step bakes in besides the state tensors: rope tables and the stream-K workspace."""

@@ -144,6 +144,13 @@ typedef struct {
 } evo_hyena_params;
 size_t evo_hyena_fwd_workspace(const evo_hyena_params* p);
 int evo_hyena_fwd(const evo_hyena_params* p, void* workspace, size_t workspace_bytes, void* stream);
+/* the same operator on a right-padded batch: row b holds lengths_dev[b] (int32, DEVICE, clamped to [0, L]) valid tokens,
+ * rows stay L apart in z and y.  state_out is the modal state after row b's own last token, fir_state_out the two z rows
+ * before lengths_dev[b] (zero when there are fewer); y past a row's length is left unwritten.  With every length == L the
+ * result is bit-identical to evo_hyena_fwd.  Mode-split scan only (head_dim 128, D % 256 == 0, EVO_B200_HYENA_VARIANT=1);
+ * halo, state_in and reuse_segment_states are rejected.  workspace: evo_hyena_fwd_ragged_workspace() bytes. */
+size_t evo_hyena_fwd_ragged_workspace(const evo_hyena_params* p);
+int evo_hyena_fwd_ragged(const evo_hyena_params* p, const int32_t* lengths_dev, void* workspace, size_t workspace_bytes, void* stream);
 
 /* decode step: engine.step_fir + step_iir.  u (B, 3D) bf16 -> y (B, D) bf16;
  * fir_state (B, 3D, 2) bf16 and state (B, D, S, 2) fp32 are updated in place. */
@@ -217,6 +224,13 @@ size_t evo_decode_attn_workspace(int B, int H, int nsplit);
 int evo_decode_attn(const void* qkv, const void* cache, void* out, const int64_t* pos, int B, int H, int hd,
                     int64_t max_seqlen, int nsplit, float softmax_scale, void* workspace, size_t workspace_bytes, void* stream);
 int evo_advance_position(int64_t* pos, int64_t delta, void* stream);
+/* the same two steps for a batch whose rows sit at different positions: pos is a DEVICE vector (B) int64 and row b's
+ * rotary row, cache slot and key range [0, pos[b]] come from pos[b].  With every entry equal they compute exactly what
+ * evo_decode_qkv_prep / evo_decode_attn compute. */
+int evo_decode_qkv_prep_rows(void* qkv, void* cache, const void* cos, const void* sin, const int64_t* pos,
+                             int B, int H, int hd, int64_t max_seqlen, void* stream);
+int evo_decode_attn_rows(const void* qkv, const void* cache, void* out, const int64_t* pos, int B, int H, int hd,
+                         int64_t max_seqlen, int nsplit, float softmax_scale, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- device-side sampler and generation loop: stripedhyena.sample.sample (evo/generation.py:162-167) and the host half
  * of the token loop (evo/generation.py:131-189) ----
@@ -242,6 +256,23 @@ int evo_sample(const void* logits, int64_t* out, int B, int V, int top_k, float 
 int evo_sample_step(const void* logits, int64_t* x, int B, int V, const evo_loop_params* loop_params_dev,
                     const int64_t* step_dev, void* stream);
 int evo_advance_counters(int64_t* a, int64_t* b, int64_t delta, void* stream);
+/* the loop for prompts of different lengths (one batch, one captured graph per step).  Row b's token at step i is
+ *   forced[b, i] while i < n_forced[b]; afterwards it is sampled (RNG counter (seed, i, b)) and recorded at column
+ *   out_cols - n_out[b] + (i - n_forced[b]) of picked (B, out_cols) int64 and kept_logits (B, out_cols, V) fp32 while
+ *   i - n_forced[b] < n_out[b]; a row past its n_forced[b] + n_out[b] steps records nothing and keeps its input token.
+ * evo_ragged_advance: *step += 1; pos[b] = start[b] + min(*step, n_forced[b] + n_out[b] - 1) (clamped at start[b]), so a
+ *   finished row keeps the position of its last step.  B <= 1024.
+ * The struct and every array it points to live in DEVICE memory. */
+typedef struct {
+  const int64_t* n_forced; const int64_t* n_out; const int64_t* start;   /* (B) each */
+  const int64_t* forced; int64_t forced_stride;                         /* (B, forced_stride) int64 or NULL */
+  int64_t* picked; float* kept_logits; int64_t out_cols;                /* (B, out_cols) int64, (B, out_cols, V) fp32; either may be NULL */
+  int32_t top_k; float top_p; float temperature;
+  uint64_t seed;
+} evo_ragged_loop_params;
+int evo_sample_step_rows(const void* logits, int64_t* x, int B, int V, const evo_ragged_loop_params* loop_params_dev,
+                         const int64_t* step_dev, void* stream);
+int evo_ragged_advance(int64_t* pos, int64_t* step, const evo_ragged_loop_params* loop_params_dev, int B, void* stream);
 
 /* (test comparators -- cuBLASLt GEMM, CUDA-core attention, bf16 add -- live in tests/support/libevo_b200_test.so,
  *  not in this library) */
